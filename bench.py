@@ -8,6 +8,12 @@ One "step" = one full pass of the hot path over one batch: `DiffusionGenerator.g
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus 8 --steps 5 --warmup 3                     # one process per GPU
     python bench.py --impl reference --steps 2 --warmup 1         # reference algorithm on the host cores
+    python bench.py --steps 5 --warmup 3 --dump-outputs DIR       # + the last timed step's images / latents as DIR/*.npy
+
+The inputs (weights, labels, noise) are seeded, so two builds run with the same arguments can be compared output for output
+on what `--dump-outputs` writes.  The latents repeat bit for bit from run to run; the decoded images do not, because the
+VAE's GroupNorm statistics are summed with shared-memory atomics in no fixed order (two runs on a B200 differed by 4e-3
+relative Frobenius), so compare images with a tolerance.
 
 Prints ONE JSON line (rank 0).  Headline keys (the contract): `value` = whole-job images/s with inputs resident in HBM;
 `e2e` = the same metric through the public API with pinned HOST inputs (H2D of labels+noise, D2H of the decoded images inside
@@ -283,6 +289,28 @@ def stock_torch_b200(dev) -> dict:
     return out
 
 
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(path: str, outputs: dict) -> None:
+    """Each output as `path/<name>.npy` in float32.  Above DUMP_BYTES in all, every output keeps the same rows of the batch,
+    a sample fixed by seed 0 and the batch size, so two runs with the same arguments write the same samples."""
+    import numpy as np
+
+    arrays = {k: v.detach().float().cpu() for k, v in outputs.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(4 * v[0].numel() for v in arrays.values())
+    keep = min(n, DUMP_BYTES // row_bytes)
+    if keep < n:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        arrays = {k: v[rows] for k, v in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v.numpy())
+    print(f"bench.py: wrote {', '.join(f'{k}{tuple(v.shape)}' for k, v in arrays.items())} (float32, {keep} of {n} "
+          f"images) to {path}", file=sys.stderr)
+
+
 def run_b200(args) -> None:
     from transformer_latent_diffusion_b200 import _lib
     from transformer_latent_diffusion_b200.denoiser import Denoiser
@@ -354,11 +382,14 @@ def run_b200(args) -> None:
     seeds_h = torch.randn(B, 4, IMG, IMG, generator=torch.Generator().manual_seed(11 + rank)).pin_memory()
     labels_d, seeds_d = labels_h.to(dev), seeds_h.to(dev)
     out_h = torch.empty(B, 3, 8 * IMG, 8 * IMG).pin_memory()
+    last = {}  # what the latest resident step returned, as DiffusionGenerator.generate returns it
 
     def step_resident():
         lat = gen.generate_latents(labels_d, n_iter=N_ITER, num_imgs=B, class_guidance=GUIDANCE, img_size=IMG,
                                    sharp_f=0, bright_f=0, exponent=1, seeds=seeds_d)
-        return vae.decode(lat * 8)[0]
+        last["images"] = vae.decode(lat * 8)[0]
+        last["latents"] = lat
+        return last["images"]
 
     def step_e2e():  # public API call with host tensors; the image comes back to (pinned) host memory
         lab = labels_h.to(dev, non_blocking=True)
@@ -380,6 +411,8 @@ def run_b200(args) -> None:
     ms_total = timed(step_resident, args.steps)
     vae_launches = vae.own_launches - vae_launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
 
@@ -576,7 +609,13 @@ def main():
     ap.add_argument("--cpu-images", type=int, default=4, help="images per CPU step (bounded sample; BASELINE.md asks for B=4)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the other BASELINE configs (512 px, 1024 px sweep, training)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the images and latents of the last timed step (rank 0) as "
+                                                          "DIR/<name>.npy, float32, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 arm computed")
     if args.impl == "reference":
         run_reference(args)
     else:
