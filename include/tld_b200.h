@@ -80,7 +80,8 @@ TLD_API int tld_denoiser_set_param(tld_denoiser* h, const char* key, const float
  * counters (fused Adam; `.data` arithmetic as in tld/train.py:55-58), so the packed copy is refreshed, not cached. */
 TLD_API int tld_denoiser_set_params_async(tld_denoiser* h, int n, const char* const* keys, const float* const* data,
                                           const int64_t* numels, void* stream);
-/* Counter bumped by every forward-like call on the handle (tld_denoiser_forward, tld_sampler_generate, tld_train_forward).
+/* Counter bumped by every forward-like call on the handle (tld_denoiser_forward, tld_sampler_generate, tld_sampler_edit,
+ * tld_train_forward).
  * The activations tld_train_backward differentiates live in per-handle buffers: the caller stores the value returned right
  * after tld_train_forward and may only run the backward while it is unchanged (tld_train_backward re-checks it). */
 TLD_API long long tld_forward_serial(tld_denoiser* h);
@@ -103,7 +104,21 @@ TLD_API int tld_denoiser_forward(tld_denoiser* h, const float* x, const float* n
 TLD_API int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seeds, float* latent_out,
                                  int num_imgs, const double* noise_levels, int n_levels, float class_guidance,
                                  float sharp_f, float bright_f, int use_ddpm_plus, void* stream);
-/* Device time of the sampling loop of the last tld_sampler_generate call (ms, CUDA events) and number of
+/* ---- image-to-image and masked inpainting on the same sampler ----------------------------------
+ * init_latent[num_imgs,C,H,W]: the known latent x0k in denoiser space (VAE latent / scale_factor); noise[num_imgs,C,H,W]:
+ * eps; mask[num_imgs,1,H,W] or NULL: 1 = regenerate, 0 = keep, clamped to [0,1] on the device (no host check).  All fp32
+ * device pointers.  noise_levels (HOST, n_levels >= 2) are the tail sig[i0:] of the generate schedule and are used
+ * verbatim; from_pure_noise = 1 means i0 == 0: the first level is forced to 0.99 and sampling starts from eps.
+ *   start:  x = eps (from_pure_noise) or sig[0]*eps + (1-sig[0])*x0k (the training corruption, tld/train.py:130)
+ *   loop:   the generate loop over the given levels (DPM-Solver++ ratios from these levels, first step first order); with a
+ *           mask, after each update to level next: x = m*x + (1-m)*(next*eps + (1-next)*x0k), the same eps every step
+ *   output: latent_out = m*x0 + (1-m)*x0k (x0 without a mask); no sharp / bright shifts.
+ * Without a mask and with from_pure_noise = 1 the result is bit-identical to tld_sampler_generate with sharp_f = bright_f = 0.
+ * Unmasked edits replay the generate step graph; masked edits use a second cached graph.  One launch more than generate. */
+TLD_API int tld_sampler_edit(tld_denoiser* h, const float* labels, const float* noise, const float* init_latent,
+                             const float* mask, float* latent_out, int num_imgs, const double* noise_levels, int n_levels,
+                             int from_pure_noise, float class_guidance, int use_ddpm_plus, void* stream);
+/* Device time of the sampling loop of the last tld_sampler_generate / tld_sampler_edit call (ms, CUDA events) and number of
  * kernel launches (graph nodes x replays + prologue) it issued. */
 TLD_API int tld_sampler_last_stats(tld_denoiser* h, float* loop_ms, int64_t* kernel_launches);
 

@@ -43,6 +43,8 @@ PROTOTYPES = {
     "tld_sampler_generate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                        C.POINTER(C.c_double), C.c_int, C.c_float, C.c_float, C.c_float, C.c_int,
                                        C.c_void_p]),
+    "tld_sampler_edit": (C.c_int, [C.c_void_p] * 6 + [C.c_int, C.POINTER(C.c_double), C.c_int, C.c_int, C.c_float, C.c_int,
+                                                    C.c_void_p]),
     "tld_sampler_last_stats": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_int64)]),
     "tld_op_gemm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                               C.c_void_p]),

@@ -202,6 +202,13 @@ static int build_params(tld_denoiser* h) {
   return dev_alloc(h, &h->staging, h->staging_elems);
 }
 
+// Both captured sampler step graphs bake in the workspace, conditioning and sampler buffer addresses: every reallocation
+// of any of them drops both.
+static void drop_step_graphs(tld_denoiser* h) {
+  if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; h->graph_batch = -1; }
+  if (h->graph_exec_masked) { cudaGraphExecDestroy(h->graph_exec_masked); h->graph_exec_masked = nullptr; h->graph_batch_masked = -1; }
+}
+
 static void free_workspace(tld_denoiser* h) {
   void* ptrs[] = {h->x_res, h->xn, h->qkv, h->hid, h->hid2, h->model_out, h->xb[0], h->xb[1], h->part[0], h->part[1]};
   for (void* p : ptrs)
@@ -209,11 +216,7 @@ static void free_workspace(tld_denoiser* h) {
   h->x_res = nullptr; h->xn = nullptr; h->qkv = nullptr; h->hid = nullptr; h->hid2 = nullptr; h->model_out = nullptr;
   h->xb[0] = h->xb[1] = nullptr; h->part[0] = h->part[1] = nullptr;
   h->ws_batch = 0;
-  if (h->graph_exec) {
-    cudaGraphExecDestroy(h->graph_exec);
-    h->graph_exec = nullptr;
-    h->graph_batch = -1;
-  }
+  drop_step_graphs(h);
 }
 
 static int ensure_workspace(tld_denoiser* h, int batch) {
@@ -245,11 +248,7 @@ static int ensure_cond(tld_denoiser* h, int rows) {
   if (h->tlevels) cudaFree(h->tlevels);
   if (h->cond_scratch) cudaFree(h->cond_scratch);
   h->ycond = nullptr; h->kv = nullptr; h->tlevels = nullptr; h->cond_scratch = nullptr;
-  if (h->graph_exec) {
-    cudaGraphExecDestroy(h->graph_exec);
-    h->graph_exec = nullptr;
-    h->graph_batch = -1;
-  }
+  drop_step_graphs(h);
   const int r = ((rows + 127) / 128) * 128;
   if (dev_alloc(h, &h->ycond, (long long)r * h->D, false)) return 1;
   if (dev_alloc(h, &h->kv, (long long)r * h->L * 2 * h->D, false)) return 1;
@@ -536,7 +535,8 @@ void tld_denoiser_destroy(tld_denoiser* h) {
   cudaDeviceSynchronize();
   free_workspace(h);
   for (void* p : h->allocs) cudaFree(p);
-  void* extra[] = {h->ycond, h->kv, h->uk, h->tlevels, h->cond_scratch, h->x_t, h->x0_prev, h->x0_out, h->step_table};
+  void* extra[] = {h->ycond, h->kv, h->uk, h->tlevels, h->cond_scratch, h->x_t, h->x0_prev, h->x0_out, h->x0k, h->eps,
+                   h->mask, h->step_table};
   for (void* p : extra)
     if (p) cudaFree(p);
   for (cudaEvent_t e : h->ev_grad)
@@ -660,20 +660,25 @@ int tld_denoiser_forward(tld_denoiser* h, const float* x, const float* noise_lev
   return run_blocks(h, batch, h->kv, kvs, h->kv + (size_t)batch * kvs, kvs, nullptr, out, st);
 }
 
-int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seeds, float* latent_out, int num_imgs,
-                         const double* noise_levels, int n_levels, float class_guidance, float sharp_f,
-                         float bright_f, int use_ddpm_plus, void* stream) {
-  TLD_CHECK(h && labels && seeds && latent_out && noise_levels, "tld_sampler_generate: null argument");
-  TLD_CHECK(num_imgs > 0, "tld_sampler_generate: num_imgs must be positive");
-  TLD_CHECK(n_levels >= 2, "tld_sampler_generate: need at least 2 noise levels");
-  TLD_CHECK(tld_denoiser_missing_params(h) == 0, "tld_sampler_generate: parameters missing");
+// What tld_sampler_edit adds to a generate call; sampler_run takes nullptr for a plain generate.
+struct EditInputs {
+  const float* init_latent;  // x0k [B,C,H,W]
+  const float* mask;         // [B,1,H,W] or nullptr (no blend: the generate step graph is replayed)
+  bool from_pure_noise;      // start from eps with the first level forced to 0.99, as generate does
+};
+
+// The body of tld_sampler_generate and tld_sampler_edit (arguments already checked).  `noise` is the initial noise of a
+// generate call, or the eps of an edit.
+static int sampler_run(tld_denoiser* h, const float* labels, const float* noise, const EditInputs* edit,
+                       float* latent_out, int num_imgs, const double* noise_levels, int n_levels, float class_guidance,
+                       float sharp_f, float bright_f, int use_ddpm_plus, void* stream) {
   TLD_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t caller = reinterpret_cast<cudaStream_t>(stream);
   cudaStream_t st = h->own_stream;
 
   // ---- multistep coefficients on the host (diffusion.py:54-57,71-81), python-float (double) arithmetic
   std::vector<double> sig(noise_levels, noise_levels + n_levels);
-  sig[0] = 0.99;
+  if (!edit || edit->from_pure_noise) sig[0] = 0.99;   // an edit from partway down the schedule uses its levels verbatim
   const int calls = (int)sig.size();
   std::vector<double> rs;
   if (use_ddpm_plus) {
@@ -696,6 +701,7 @@ int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seed
       sc.dsig = (float)(cur - next);
       sc.next = (float)next;
       sc.cur = (float)cur;
+      sc.one_minus_next = (float)(1.0 - next);
       if (i > 0 && use_ddpm_plus) {
         sc.c1 = (float)(1.0 + 1.0 / (2.0 * rs[i - 1]));
         sc.c2 = (float)(1.0 / (2.0 * rs[i - 1]));
@@ -712,25 +718,28 @@ int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seed
 
   // ---- buffers
   const int Beff = 2 * num_imgs;
-  const long long img_elems = (long long)num_imgs * h->C * h->img * h->img;
+  const long long hw = (long long)h->img * h->img;
+  const long long img_elems = (long long)num_imgs * h->C * hw;
   if (ensure_workspace(h, Beff) || ensure_cond(h, calls + Beff)) return 1;
   ++h->fwd_serial;
   if (num_imgs > h->sampler_batch) {
     TLD_CUDA_OK(cudaDeviceSynchronize());
-    float** bufs[] = {&h->x_t, &h->x0_prev, &h->x0_out};
+    float** bufs[] = {&h->x_t, &h->x0_prev, &h->x0_out, &h->x0k, &h->eps};
     for (float** b : bufs) {
       if (*b) cudaFree(*b);
       if (dev_alloc(h, b, img_elems, false)) return 1;
     }
+    if (h->mask) cudaFree(h->mask);
+    if (dev_alloc(h, &h->mask, num_imgs * hw, false)) return 1;
     h->sampler_batch = num_imgs;
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; h->graph_batch = -1; }
+    drop_step_graphs(h);
   }
   if (calls > h->step_table_cap) {
     TLD_CUDA_OK(cudaDeviceSynchronize());
     if (h->step_table) cudaFree(h->step_table);
     if (dev_alloc(h, &h->step_table, calls, false)) return 1;
     h->step_table_cap = calls;
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; h->graph_batch = -1; }
+    drop_step_graphs(h);
   }
 
   // ---- per-call host tables go through a library-owned pinned buffer: the copies are asynchronous and the host never
@@ -755,7 +764,18 @@ int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seed
   TLD_CUDA_OK(cudaMemcpyAsync(h->tlevels, reinterpret_cast<char*>(h->pin_host) + table_bytes, tl_bytes, cudaMemcpyHostToDevice, st));
   TLD_CUDA_OK(cudaEventRecord(h->ev_tables, st));
   TLD_CUDA_OK(cudaMemsetAsync(h->step_ptr, 0, sizeof(int), st));
-  TLD_CUDA_OK(cudaMemcpyAsync(h->x_t, seeds, sizeof(float) * img_elems, cudaMemcpyDeviceToDevice, st));
+  if (!edit) {
+    TLD_CUDA_OK(cudaMemcpyAsync(h->x_t, noise, sizeof(float) * img_elems, cudaMemcpyDeviceToDevice, st));
+  } else {
+    // the inputs go to handle-owned buffers: the masked step graph reads them at baked-in addresses
+    TLD_CUDA_OK(cudaMemcpyAsync(h->eps, noise, sizeof(float) * img_elems, cudaMemcpyDeviceToDevice, st));
+    TLD_CUDA_OK(cudaMemcpyAsync(h->x0k, edit->init_latent, sizeof(float) * img_elems, cudaMemcpyDeviceToDevice, st));
+    if (edit->mask)
+      TLD_CUDA_OK(cudaMemcpyAsync(h->mask, edit->mask, sizeof(float) * num_imgs * hw, cudaMemcpyDeviceToDevice, st));
+    // x_t = sig[0]*eps + (1-sig[0])*x0k (the training corruption, tld/train.py:130), or eps from pure noise
+    if (launch_edit_start(h->x_t, h->eps, h->x0k, (float)sig[0], (float)(1.0 - sig[0]), edit->from_pure_noise, img_elems, st))
+      return 1;
+  }
 
   // ---- conditioning hoisted out of the loop: the noise token depends only on the step, the label token only
   // on the sample (SURVEY.md §2.2 K13/K22).  rows [0, 2B): label tokens; rows [2B, 2B+calls): noise tokens.  The label
@@ -773,35 +793,63 @@ int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seed
   const float* kv1 = h->kv;
   const float* kv0 = h->kv + (size_t)Beff * kvs;
 
-  // ---- one diffusion step = one CUDA graph (embed of cat[x,x] -> L blocks -> out-proj -> CFG + update)
-  if (!h->graph_exec || h->graph_batch != num_imgs || h->graph_epoch != g_option_epoch) {
-    if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
+  // ---- one diffusion step = one CUDA graph (embed of cat[x,x] -> L blocks -> out-proj -> CFG + update).  A masked edit has
+  // its own graph, which differs in the update kernel only; an unmasked edit replays the generate graph.
+  const bool masked = edit && edit->mask;
+  cudaGraphExec_t& graph_exec = masked ? h->graph_exec_masked : h->graph_exec;
+  int& graph_batch = masked ? h->graph_batch_masked : h->graph_batch;
+  int& graph_epoch = masked ? h->graph_epoch_masked : h->graph_epoch;
+  if (!graph_exec || graph_batch != num_imgs || graph_epoch != g_option_epoch) {
+    if (graph_exec) { cudaGraphExecDestroy(graph_exec); graph_exec = nullptr; }
     cudaGraph_t graph = nullptr;
     TLD_CUDA_OK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
     int rc = launch_embed(h->x_t, num_imgs, Beff, h->C, h->img, h->patch, h->D, h->emb, h->x_res, st);
     if (!rc) rc = run_blocks(h, Beff, kv0, kvs /*row = *step_ptr*/, kv1, kvs, h->step_ptr, h->model_out, st, num_imgs);
     if (!rc)
       rc = launch_cfg_update(h->model_out, h->x_t, h->x0_prev, h->x0_out, h->step_table, h->step_ptr, num_imgs, h->C,
-                             h->img * h->img, st);
+                             h->img * h->img, st, h->x0k, h->eps, masked ? h->mask : nullptr);
     if (!rc) rc = launch_advance_step(h->step_ptr, st);
     cudaError_t ce = cudaStreamEndCapture(st, &graph);
     if (rc) { if (graph) cudaGraphDestroy(graph); return 1; }
     TLD_CUDA_OK(ce);
-    ce = cudaGraphInstantiate(&h->graph_exec, graph, 0);
+    ce = cudaGraphInstantiate(&graph_exec, graph, 0);
     cudaGraphDestroy(graph);
     TLD_CUDA_OK(ce);
-    h->graph_batch = num_imgs;
-    h->graph_epoch = g_option_epoch;
+    graph_batch = num_imgs;
+    graph_epoch = g_option_epoch;
   }
   TLD_CUDA_OK(cudaEventRecord(h->ev_t0, st));
-  for (int i = 0; i < calls; ++i) TLD_CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
+  for (int i = 0; i < calls; ++i) TLD_CUDA_OK(cudaGraphLaunch(graph_exec, st));
   TLD_CUDA_OK(cudaEventRecord(h->ev_t1, st));
   TLD_CUDA_OK(cudaMemcpyAsync(latent_out, h->x0_out, sizeof(float) * img_elems, cudaMemcpyDeviceToDevice, st));
   TLD_CUDA_OK(cudaEventRecord(h->ev_out, st));
   TLD_CUDA_OK(cudaStreamWaitEvent(caller, h->ev_out, 0));
-  h->last_launches = (long long)calls * (kernels_per_forward(h) + 2) + 3 + (use_fused_xattn(h) ? h->L : 0);
+  h->last_launches = (long long)calls * (kernels_per_forward(h) + 2) + 3 + (use_fused_xattn(h) ? h->L : 0) + (edit ? 1 : 0);
   h->last_loop_ms = -1.f;
   return 0;
+}
+
+int tld_sampler_generate(tld_denoiser* h, const float* labels, const float* seeds, float* latent_out, int num_imgs,
+                         const double* noise_levels, int n_levels, float class_guidance, float sharp_f,
+                         float bright_f, int use_ddpm_plus, void* stream) {
+  TLD_CHECK(h && labels && seeds && latent_out && noise_levels, "tld_sampler_generate: null argument");
+  TLD_CHECK(num_imgs > 0, "tld_sampler_generate: num_imgs must be positive");
+  TLD_CHECK(n_levels >= 2, "tld_sampler_generate: need at least 2 noise levels");
+  TLD_CHECK(tld_denoiser_missing_params(h) == 0, "tld_sampler_generate: parameters missing");
+  return sampler_run(h, labels, seeds, nullptr, latent_out, num_imgs, noise_levels, n_levels, class_guidance, sharp_f,
+                     bright_f, use_ddpm_plus, stream);
+}
+
+int tld_sampler_edit(tld_denoiser* h, const float* labels, const float* noise, const float* init_latent, const float* mask,
+                     float* latent_out, int num_imgs, const double* noise_levels, int n_levels, int from_pure_noise,
+                     float class_guidance, int use_ddpm_plus, void* stream) {
+  TLD_CHECK(h && labels && noise && init_latent && latent_out && noise_levels, "tld_sampler_edit: null argument");
+  TLD_CHECK(num_imgs > 0, "tld_sampler_edit: num_imgs must be positive");
+  TLD_CHECK(n_levels >= 2, "tld_sampler_edit: need at least 2 noise levels");
+  TLD_CHECK(tld_denoiser_missing_params(h) == 0, "tld_sampler_edit: parameters missing");
+  const EditInputs edit{init_latent, mask, from_pure_noise != 0};
+  return sampler_run(h, labels, noise, &edit, latent_out, num_imgs, noise_levels, n_levels, class_guidance, 0.f, 0.f,
+                     use_ddpm_plus, stream);
 }
 
 int tld_sampler_last_stats(tld_denoiser* h, float* loop_ms, int64_t* kernel_launches) {

@@ -133,11 +133,18 @@ struct StepCoef {  // one entry per model call of the sampler (device table)
   float dsig, next, cur;  // x_t = (dsig*D + next*x_t)/cur
   int is_final;        // last model call: emit x0 (+ channel shifts), no x_t update
   float sharp, bright;
+  float one_minus_next;   // masked edit: the kept region of x_t is reset to next*eps + one_minus_next*x0k
 };
-// model_out[2B,...] (cond first, uncond second) -> CFG combine -> multistep update of x_t / x0_prev / x0_out
+// model_out[2B,...] (cond first, uncond second) -> CFG combine -> multistep update of x_t / x0_prev / x0_out.
+// mask != nullptr (masked edit, mask [B,1,H,W] clamped to [0,1], 1 = regenerate): after each update
+// x_t = m*x_t + (1-m)*(next*eps + (1-next)*x0k), and the final x0_out = m*x0 + (1-m)*x0k
 int launch_cfg_update(const float* model_out, float* x_t, float* x0_prev, float* x0_out, const StepCoef* table,
-                      const int* step_ptr, int B, int C, int hw, cudaStream_t st);
+                      const int* step_ptr, int B, int C, int hw, cudaStream_t st, const float* x0k = nullptr,
+                      const float* eps = nullptr, const float* mask = nullptr);
 int launch_advance_step(int* step_ptr, cudaStream_t st);
+// start state of an edit: x_t = eps (from_noise) or s0*eps + one_minus_s0*x0k, n elements
+int launch_edit_start(float* x_t, const float* eps, const float* x0k, float s0, float one_minus_s0, int from_noise,
+                      long long n, cudaStream_t st);
 
 // 3x3 'same' conv as implicit GEMM: x NHWC bf16, w bf16 [Cout, 9*Cin] with K order (ky,kx,cin), bias fp32 or null
 int launch_conv3x3(const bf16* x, const bf16* w, const float* bias, bf16* out, int B, int H, int W, int Cin, int Cout,

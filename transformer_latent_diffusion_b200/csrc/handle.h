@@ -74,6 +74,8 @@ struct tld_denoiser {
   cudaStream_t own_stream = nullptr;
   cudaEvent_t ev_in = nullptr, ev_out = nullptr, ev_t0 = nullptr, ev_t1 = nullptr;
   float *x_t = nullptr, *x0_prev = nullptr, *x0_out = nullptr;
+  float *x0k = nullptr, *eps = nullptr;  // tld_sampler_edit: known latent and noise [B,C,H,W]
+  float* mask = nullptr;                 // tld_sampler_edit: [B,1,H,W], 1 = regenerate
   int sampler_batch = 0;
   StepCoef* step_table = nullptr;
   int step_table_cap = 0;
@@ -81,13 +83,16 @@ struct tld_denoiser {
   cudaGraphExec_t graph_exec = nullptr;
   int graph_batch = -1;
   int graph_epoch = -1;          // tld_set_option epoch the graph was captured under
+  cudaGraphExec_t graph_exec_masked = nullptr;  // the same step with the masked update (both bake in the sampler buffers)
+  int graph_batch_masked = -1;
+  int graph_epoch_masked = -1;
   void* pin_host = nullptr;      // pinned staging of the per-call step table + noise levels
   size_t pin_cap = 0;
   cudaEvent_t ev_tables = nullptr;  // the previous call's table copies have left pin_host
   float last_loop_ms = 0.f;
   long long last_launches = 0;
 
-  // every forward-like call (forward, sampler, training forward) bumps fwd_serial; train_serial remembers the one whose
+  // every forward-like call (forward, sampler generate / edit, training forward) bumps fwd_serial; train_serial remembers the one whose
   // activations the training buffers (and x_res) currently hold, so a backward after any later forward is refused
   long long fwd_serial = 0;
   long long train_serial = -1;

@@ -1102,17 +1102,24 @@ int launch_outproj(const float* x, const float* w, const float* b, float* out, i
 // --------------------------------------------------------------------------------------------
 // CFG combine + DPM-Solver++(2M)/DDIM update (diffusion.py:66-89,122-125), coefficients from a device table.
 // Separate rounded multiplies/adds (no FMA contraction) to follow the eager reference op by op.
+// MASKED (masked edit): the kept region (mask 0) of x_t is reset to the known latent re-noised to the next level with the
+// same eps after every update, and the final prediction keeps the known latent there; x0_prev keeps the unblended x0.
 // --------------------------------------------------------------------------------------------
+template <bool MASKED>
 __global__ void __launch_bounds__(256) cfg_update_kernel(const float* __restrict__ mo, float* __restrict__ x_t,
                                                          float* __restrict__ x0_prev, float* __restrict__ x0_out,
                                                          const StepCoef* __restrict__ table,
-                                                         const int* __restrict__ step_ptr, int B, int C, int hw) {
+                                                         const int* __restrict__ step_ptr, int B, int C, int hw,
+                                                         const float* __restrict__ x0k, const float* __restrict__ eps,
+                                                         const float* __restrict__ mask) {
   pdl_launch_dependents();
   pdl_wait();
   const StepCoef sc = table[*step_ptr];
   const long long n = (long long)B * C * hw;
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
+  float m = 1.f;
+  if constexpr (MASKED) m = fminf(fmaxf(mask[(i / ((long long)C * hw)) * hw + i % hw], 0.f), 1.f);  // one value per pixel
   const float c = mo[i], u = mo[n + i];
   const float x0 = __fadd_rn(__fmul_rn(sc.guidance, c), __fmul_rn(sc.one_minus_g, u));
   if (sc.is_final) {
@@ -1120,14 +1127,27 @@ __global__ void __launch_bounds__(256) cfg_update_kernel(const float* __restrict
     float v = x0;
     if (ch == 3) v = __fadd_rn(v, sc.sharp);
     if (ch == 0) v = __fadd_rn(v, sc.bright);
+    if constexpr (MASKED) v = __fadd_rn(__fmul_rn(m, v), __fmul_rn(__fsub_rn(1.f, m), x0k[i]));
     x0_out[i] = v;
     return;
   }
   float d = x0;
   if (sc.c2 != 0.f) d = __fsub_rn(__fmul_rn(sc.c1, x0), __fmul_rn(sc.c2, x0_prev[i]));
   const float num = __fadd_rn(__fmul_rn(sc.dsig, d), __fmul_rn(sc.next, x_t[i]));
-  x_t[i] = __fdiv_rn(num, sc.cur);
+  float xn = __fdiv_rn(num, sc.cur);
+  if constexpr (MASKED) {
+    const float kept = __fadd_rn(__fmul_rn(sc.next, eps[i]), __fmul_rn(sc.one_minus_next, x0k[i]));
+    xn = __fadd_rn(__fmul_rn(m, xn), __fmul_rn(__fsub_rn(1.f, m), kept));
+  }
+  x_t[i] = xn;
   x0_prev[i] = x0;
+}
+
+__global__ void edit_start_kernel(float* __restrict__ x_t, const float* __restrict__ eps, const float* __restrict__ x0k,
+                                  float s0, float one_minus_s0, int from_noise, long long n) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  x_t[i] = from_noise ? eps[i] : __fadd_rn(__fmul_rn(s0, eps[i]), __fmul_rn(one_minus_s0, x0k[i]));
 }
 
 __global__ void advance_step_kernel(int* step_ptr) {
@@ -1137,10 +1157,20 @@ __global__ void advance_step_kernel(int* step_ptr) {
 }
 
 int launch_cfg_update(const float* model_out, float* x_t, float* x0_prev, float* x0_out, const StepCoef* table,
-                      const int* step_ptr, int B, int C, int hw, cudaStream_t st) {
+                      const int* step_ptr, int B, int C, int hw, cudaStream_t st, const float* x0k, const float* eps,
+                      const float* mask) {
   const long long n = (long long)B * C * hw;
-  return launch_pdl(cfg_update_kernel, dim3(int((n + 255) / 256)), dim3(256), 0, st, model_out, x_t, x0_prev, x0_out, table, step_ptr,
-                    B, C, hw);
+  if (mask)
+    return launch_pdl(cfg_update_kernel<true>, dim3(int((n + 255) / 256)), dim3(256), 0, st, model_out, x_t, x0_prev, x0_out,
+                      table, step_ptr, B, C, hw, x0k, eps, mask);
+  return launch_pdl(cfg_update_kernel<false>, dim3(int((n + 255) / 256)), dim3(256), 0, st, model_out, x_t, x0_prev, x0_out,
+                    table, step_ptr, B, C, hw, nullptr, nullptr, nullptr);
+}
+int launch_edit_start(float* x_t, const float* eps, const float* x0k, float s0, float one_minus_s0, int from_noise,
+                      long long n, cudaStream_t st) {
+  edit_start_kernel<<<int((n + 255) / 256), 256, 0, st>>>(x_t, eps, x0k, s0, one_minus_s0, from_noise, n);
+  TLD_CUDA_OK(cudaGetLastError());
+  return 0;
 }
 int launch_advance_step(int* step_ptr, cudaStream_t st) {
   return launch_pdl(advance_step_kernel, dim3(1), dim3(1), 0, st, step_ptr);
